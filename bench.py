@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SAM-PT hot path throughput on B200 (contract: see the task brief / DESIGN.md §measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C1|...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2|C1|...] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (PIPS track -> SAM ViT encode -> prompt+mask decode with 12 refinements) over one
 synthetic clip.  Headline workload = BASELINE config C2: 50 frames 480x854, SAM ViT-H + PIPS, 1 mask x 8 positive points.
@@ -176,8 +176,10 @@ def run_ours(args):
         for i in range(args.steps):
             flush.fill_(i & 0xFF)
             ev[i][0].record()
-            step_resident(frames_dev, q_dev)
+            last = step_resident(frames_dev, q_dev)
             ev[i][1].record()
+            if i + 1 < args.steps or not args.dump_outputs:
+                del last   # only the last step's outputs stay alive, and only for --dump-outputs
         barrier()
     ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = ctx.launch_count() - launches0
@@ -239,9 +241,49 @@ def run_ours(args):
         }
         if breakdown:
             line["breakdown_ms"] = breakdown
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(zip(("logits", "scores_per_frame", "trajectories", "visibilities"), last)))
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE_ELEMS = 1 << 22   # 16 MiB of float32, written twice (values and -inf marks)
+
+
+def dump_outputs(path, outputs):
+    """Writes the tensors the last timed resident step returned as `path/<name>.npy` (float32; float64 stays float64), so that
+    two builds can be compared output for output on the same seeded inputs.  A tensor of more than DUMP_SAMPLE_ELEMS elements
+    (the logits of the 50- and 100-frame configurations) is written as `<name>_sample.npy`: the flat elements at DUMP_SAMPLE_ELEMS
+    indices drawn without replacement by a CPU generator seeded with 0, in increasing index order, hence the same elements
+    on every run of the same configuration.  With several ranks (--mgpu-mode clip_per_gpu) only rank 0's clip (seed 72) is
+    written.
+
+    A frame on which every tracked point of a mask is invisible gets no SAM call: its logits and its score are -inf, as in the
+    reference.  The files hold finite numbers only: a -inf is written as 0 in `<name>.npy` and marked by 1 in
+    `<name>_neginf.npy` (written for every tensor), so a comparison sees both the values and which entries were skipped
+    without an infinite or huge stand-in swamping the differences.  NaN or +inf is never produced and raises."""
+    import numpy as np
+    arrays = {}
+    for name, t in outputs.items():
+        t = t.detach()
+        t = t if t.dtype == torch.float64 else t.float()
+        if t.numel() > DUMP_SAMPLE_ELEMS:
+            g = torch.Generator(device="cpu").manual_seed(0)
+            idx = torch.randperm(t.numel(), generator=g)[:DUMP_SAMPLE_ELEMS].sort().values
+            name, t = name + "_sample", t.reshape(-1)[idx.to(t.device)]
+        neginf = torch.isneginf(t)
+        if not torch.isfinite(t[~neginf]).all():
+            raise RuntimeError(f"--dump-outputs: {name} holds NaN or +inf")
+        arrays[name] = t.masked_fill(neginf, 0).cpu().numpy()
+        arrays[name + "_neginf"] = neginf.to(t.dtype).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES} byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def run_ours_frame_sharded(args, model, dev, rank, world, local):
@@ -681,7 +723,16 @@ def main():
     ap.add_argument("--kernel-table", default=None, help="write a per-kernel time table of one step (CUPTI) to this path")
     ap.add_argument("--mgpu-mode", default="frame_shard", choices=["frame_shard", "clip_per_gpu"])
     ap.add_argument("--clips-per-step", type=int, default=0, help="N > 1: clips per step (default: one per rank; C5: a single clip)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the run, write what the last timed resident step returned to DIR/<name>.npy (float32, at most 64 MiB; "
+                         "tensors over 4 Mi elements as a fixed seeded sample, -inf as 0 plus a <name>_neginf.npy mark)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm computes no outputs here")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1 and args.mgpu_mode == "frame_shard":
+        ap.error("--dump-outputs needs whole clips per rank: use --mgpu-mode clip_per_gpu")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,12 +1,11 @@
-"""CPU, build container only (skipped where /root/reference is absent): the reference's UNMODIFIED Hydra YAMLs resolve to
-this repo's drop-in classes and construct the full SamPt object tree (SURVEY §8b boundary contract)."""
+"""CPU: the reference's UNMODIFIED Hydra YAMLs (its configs/model tree, stored under tests/golden/reference_configs) resolve
+to this repo's drop-in classes and construct the full SamPt object tree (SURVEY §8b boundary contract)."""
 import os
 
 import pytest
 import torch
 
-REF_CFG = "/root/reference/configs"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference configs only exist in the build container")
+REF_CFG = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs")
 
 
 def test_reference_yaml_instantiates_dropin(tmp_path):

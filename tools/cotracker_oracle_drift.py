@@ -1,5 +1,6 @@
-import sys, torch, time
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/sam-pt_b200')
+import os, sys, torch, time
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'sam-pt_b200'))
 from oracle import cotracker_ref as R
 from sampt_b200 import synth
 def run(threads, scale=None, P=64):
